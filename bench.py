@@ -316,6 +316,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the extra BASELINE.json configurations (ViT-L/16-384, q8_0)")
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (probabilities, top-5 indices and "
+                    "values) as DIR/<name>.npy")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -403,6 +405,12 @@ def main():
         ms_local, clocks = timed_region(args.steps)
         clocks["remeasured_after"] = first.get("reasons", [])
     launches_per_step = model.last_launch_count()
+    if args.dump_outputs:
+        # the inputs are seeded, so two builds given the same arguments can be compared output for output
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        suffix = "" if world == 1 else "_rank%d" % rank
+        for name, arr in (("probs", d_probs), ("topk_idx", d_idx), ("topk_prob", d_val)):
+            np.save(os.path.join(args.dump_outputs, name + suffix + ".npy"), arr.cpu().numpy().astype(np.float32))
     t = torch.tensor([ms_local], device="cuda", dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -546,7 +554,10 @@ def main():
                 run_extra_config(eng, L, gf, torch, "vit_base_patch16_224 q8_0 model file (weights dequantised to f16 at upload), batch=256",
                                  "base", "q8_0", 256, 10, 3, os.path.join(gd, "base_q8_0.npz"), peaks, local_rank, stream),
             ]
-        if world == 1 and not args.no_cpu_baseline:
+        from oracle import ref
+        if world == 1 and not args.no_cpu_baseline and not ref.available():
+            line["cpu_baseline"] = None   # the compiled reference (oracle/_ref) is only built where its sources are present
+        elif world == 1 and not args.no_cpu_baseline:
             nproc = host_threads()
             rate, nt, dt, tried = cpu_reference_rate(8, thread_candidates())
             line["cpu_baseline"] = {"value": rate, "unit": "images/s", "cores": nt, "kind": "reference",

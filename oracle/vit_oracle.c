@@ -56,11 +56,11 @@ static float g_tab_gelu[1 << 16];
 static float g_tab_exp[1 << 16];
 static int g_tab_init = 0;
 
-/* ggml.c:1414-1424 ggml_gelu_f32 (tanh form, NOT erf) */
+/* ggml.c:1414-1424 ggml_gelu_f32 (tanh form, NOT erf); the reference build contracts 1 + A*x*x into one fma */
 static inline float gelu_f32(float x) {
     const float GELU_COEF_A = 0.044715f;
     const float SQRT_2_OVER_PI = 0.79788456080286535587989211986876f;
-    return 0.5f * x * (1.0f + tanhf(SQRT_2_OVER_PI * x * (1.0f + GELU_COEF_A * x * x)));
+    return 0.5f * x * (1.0f + tanhf(SQRT_2_OVER_PI * x * fmaf(GELU_COEF_A * x, x, 1.0f)));
 }
 
 static void init_tables(void) {
@@ -88,9 +88,10 @@ static inline float reduce_4x8(const float *s) {
 /* ggml.c:1163-1198 ggml_vec_dot_f32 and ggml.c:1200-1236 ggml_vec_dot_f16 (operands already
  * widened to f32 -- f16*f16 products are exact in f32, so vfmadd on widened values is the same
  * arithmetic).  `dbl_tail`: the f16 kernel accumulates leftovers in double; the f32 kernel adds
- * them in float, in order, as separate multiply and add (gcc vectorises the multiplies of that
- * loop and keeps the adds sequential, so no fused multiply-add there -- checked in the
- * disassembly of the reference build and pinned bit-for-bit by tests/test_oracle.py). */
+ * them in float, in order: gcc vectorises the multiplies of that loop 8 and then 4 at a time and
+ * keeps the adds sequential, and its scalar epilogue for the last (n - np) % 4 terms is a fused
+ * multiply-add (checked in the disassembly of the reference build, gcc 13, and pinned bit-for-bit
+ * by tests/test_oracle.py). */
 /* Experiment knob (tests/bench never set it): 0 = the reference's arithmetic (default, bit-exact);
  * 1 = same rounding points but dot products accumulated in double ("any other correct implementation");
  * 2 = 1 + q,k,v rounded to f16 before attention; 3 = 1 + only v rounded to f16; 4 = 1 + only q,k rounded to f16;
@@ -132,7 +133,9 @@ static float dot_ggml(int n, const float *x, const float *y, int dbl_tail) {
         for (int i = np; i < n; ++i) sd += (double)(x[i] * y[i]);
         return (float)sd;
     }
-    for (int i = np; i < n; ++i) r = r + x[i] * y[i];
+    const int nf = n - ((n - np) & 3);
+    for (int i = np; i < nf; ++i) r = r + x[i] * y[i];
+    for (int i = nf; i < n; ++i) r = fmaf(x[i], y[i], r);
     return r;
 }
 

@@ -4,10 +4,12 @@ import importlib.util
 import os
 import subprocess
 import sys
+import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG_DIR = os.path.join(ROOT, "vit.cpp_b200")
-CACHE = os.environ.get("VITB200_CACHE", os.path.join(ROOT, ".cache"))
+# generated model files live outside the tree (which may be read-only) and are shared by later runs of the same user
+CACHE = os.environ.get("VITB200_CACHE", os.path.join(tempfile.gettempdir(), f"vitb200-cache-{os.getuid()}"))
 
 
 def load_pkg():
