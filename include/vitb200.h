@@ -180,6 +180,12 @@ int vitb200_test_gemm(int device, int M, int N, int K, int epilogue, const uint1
  * ggml.c:8959-9008): x float32 [rows][D] -> y float32 [rows][D] holding the f16 results (the next GEMM's A operand) widened. */
 int vitb200_test_layernorm(int device, int rows, int D, const float *x, const float *w, const float *b, float eps, float *y);
 
+/* Stand-alone run of the final soft-max + top-k (reference vit.cpp:931 + the sorted predictions of vit.cpp:1047-1057) through the
+ * forward's own launcher: logits = float32 [R][ldl] (host), of which the first C columns of every row are read; probs = float32 [R][C]
+ * with the reference's f16-exp semantics; idx / val = [R][k], probabilities descending, index ascending on ties, entries past C are
+ * (-1, 0).  0 <= k <= 16 (the forward's limit); idx / val may be NULL when k == 0. */
+int vitb200_test_softmax_topk(int device, int R, int C, int ldl, const float *logits, int k, float *probs, int32_t *idx, float *val);
+
 /* Prototype of the reference's q8_0 x q8_0 linear layer on the INTEGER tensor cores (tcgen05.mma kind::i8, one K = 32 MMA per
  * q8_0 block; csrc/gemm_q8_tcgen05.cuh).  Replaces, for one layer, quantize_row_q8_0 (reference ggml-quants.c:702-790: the f32
  * activation rows x [M][K] are quantised on the device, bit for bit as the reference does) + ggml_vec_dot_q8_0_q8_0

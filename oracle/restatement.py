@@ -166,3 +166,40 @@ def linear_q8_0(x, w_blocks, bias):
     xd = np.empty((T, K // 32), np.float32)
     lib().vo_linear_q8_0(T, N, K, w_blocks.ctypes.data, bias.ctypes.data, x.ctypes.data, y.ctypes.data, xd.ctypes.data, xq.ctypes.data)
     return y, xq, xd
+
+
+def preprocess_levels(rgb_u8, S: int, bilinear: bool = False):
+    """numpy restatement of vit_image_preprocess's resize (reference vit.cpp:130-287) up to the u8 levels it rounds to before
+    normalising: HxWx3 uint8 -> SxSx3 uint8.  Same sampling positions, taps and float32 roundings as the reference, but without the
+    fused multiply-adds its compiled build contains, so an occasional level differs by one: the preprocess fixture stores the
+    reference's levels as a residual against this prediction, which keeps it small (tests/golden/make_golden_ref.py)."""
+    img = np.asarray(rgb_u8, np.uint8).astype(np.float32)
+    ny, nx = img.shape[:2]
+    f32 = np.float32
+    j = np.arange(S, dtype=np.float32)
+    if bilinear:
+        xs_, ys_ = f32(nx) / f32(S), f32(ny) / f32(S)
+        sx, sy = (j + f32(0.5)) * xs_ - f32(0.5), (j + f32(0.5)) * ys_ - f32(0.5)
+        x0, y0 = np.maximum(0, np.floor(sx).astype(np.int64)), np.maximum(0, np.floor(sy).astype(np.int64))
+        x1, y1 = np.minimum(x0 + 1, nx - 1), np.minimum(y0 + 1, ny - 1)
+        dx, dy = (sx - x0.astype(np.float32))[None, :, None], (sy - y0.astype(np.float32))[:, None, None]
+        v0 = img[y0][:, x0] * (f32(1) - dx) + img[y0][:, x1] * dx
+        v1 = img[y1][:, x0] * (f32(1) - dx) + img[y1][:, x1] * dx
+        v = v0 * (f32(1) - dy) + v1 * dy
+    else:
+        def cubic(p0, p1, p2, p3, t):
+            d0, d2, d3 = (p0 - p1).astype(np.float64), (p2 - p1).astype(np.float64), (p3 - p1).astype(np.float64)
+            a1 = (-1.0 / 3 * d0 + d2 - 1.0 / 6 * d3).astype(np.float32)
+            a2 = (1.0 / 2 * d0 + 1.0 / 2 * d2).astype(np.float32)
+            a3 = (-1.0 / 6 * d0 - 1.0 / 2 * d2 + 1.0 / 6 * d3).astype(np.float32)
+            return p1 + a1 * t + a2 * t * t + a3 * t * t * t
+        tx, ty = f32(nx) / f32(S), f32(ny) / f32(S)
+        fx, fy = tx * j, ty * j
+        x, y = fx.astype(np.int64), fy.astype(np.int64)
+        dx, dy = (fx - x.astype(np.float32))[None, :, None], (fy - y.astype(np.float32))[:, None, None]
+        cols = [np.clip(x + o, 0, nx - 1) for o in (-1, 0, 1, 2)]
+        rows = [img[np.clip(y + o, 0, ny - 1)] for o in (-1, 0, 1, 2)]          # [S][nx][3] each
+        C = [cubic(*(r[:, c] for c in cols), dx) for r in rows]
+        v = cubic(*C, dy)
+    r = np.sign(v) * np.floor(np.abs(v) + f32(0.5))                            # roundf: half away from zero
+    return np.clip(r, 0, 255).astype(np.uint8)

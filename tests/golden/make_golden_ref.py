@@ -6,7 +6,11 @@ they compare against the reference without needing it at test time.  Run where o
                  and bf16-weight parity of the engine, the u8 -> preprocess -> predict pipeline), the reference's primitive ops (GELU
                  table on every finite f16, soft-max rows, f16 rounding, norm), ggml's block quantisers + dequantisers on a seeded
                  vector, and the sha256 of the reference quantize binary's q8_0 files.  Outputs that the tests only compare bit for
-                 bit are stored as the sha256 of their float32 bytes (digest()), which keeps the fixture small."""
+                 bit are stored as the sha256 of their float32 bytes (digest()), which keeps the fixture small.
+  preprocess_ref.npz  the reference's bicubic and bilinear vit_image_preprocess of ggml_file.preprocess_test_images() resized to
+                 S = 64, 56 and 224, as the u8 levels it rounds to before normalising (the encoding is checked to be lossless against
+                 its float output).  `{bicubic,bilinear}_{S}` ([image][S][S][3] int8) holds each level minus the numpy restatement's
+                 prediction of it (restatement.preprocess_levels): mostly zeros, which keeps noise images at S = 224 small."""
 import ctypes as C
 import hashlib
 import os
@@ -19,7 +23,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from tests.util import gf, model_path  # noqa: E402
-from oracle import ref  # noqa: E402
+from oracle import ref, restatement as rs  # noqa: E402
 
 BIT_EXACT = [("micro", "f16"), ("micro14", "f16"), ("micro", "f32"), ("micro", "q8_0"), ("tiny", "f16")]
 
@@ -105,13 +109,50 @@ def forwards(out):
     m.close()
 
 
+PREPROCESS_SIZES = (("micro", 64), ("micro14", 56), ("tiny", 224))   # (model whose img_size the reference resizes to, S)
+PRE_MEAN = np.array([123.675, 116.280, 103.530], np.float32)          # vit.cpp:233-234
+PRE_STD = np.array([58.395, 57.120, 57.375], np.float32)
+
+
+def preprocess(out):
+    """The reference's bicubic and bilinear vit_image_preprocess of gf.preprocess_test_images() at every S, as the u8 levels the
+    reference rounds to before normalising ((level - mean_c) / std_c in float32 must give back its output bit for bit), stored as
+    residuals against rs.preprocess_levels."""
+    imgs = gf.preprocess_test_images()
+    for cfg, S in PREPROCESS_SIZES:
+        m = ref.RefModel(model_path(cfg, "f16"))
+        assert m.img == S
+        for mode, bilinear in (("bicubic", False), ("bilinear", True)):
+            levels = []
+            for im in imgs:
+                ny, nx = im.shape[:2]
+                if bilinear:   # the reference's output extent, int(n / (n / (float)S) + 0.5f), must be S (vit.cpp:143-144)
+                    for n in (nx, ny):
+                        assert int(np.float32(n) / (np.float32(n) / np.float32(S)) + np.float32(0.5)) == S, (n, S)
+                want = m.preprocess(im, bilinear=bilinear)
+                lv = np.clip(np.rint(want * PRE_STD + PRE_MEAN), 0, 255).astype(np.uint8)
+                back = (lv.astype(np.float32) - PRE_MEAN) / PRE_STD
+                assert np.array_equal(back.view(np.uint32), want.view(np.uint32)), (cfg, mode, im.shape)
+                res = lv.astype(np.int16) - rs.preprocess_levels(im, S, bilinear)
+                assert np.abs(res).max() <= 127
+                levels.append(res.astype(np.int8))
+            out[f"{mode}_{S}"] = np.stack(levels)
+        m.close()
+
+
 def main():
+    here = os.path.dirname(os.path.abspath(__file__))
     out = {}
     primitives(out)
     dequant(out)
     quantize_sha(out)
     forwards(out)
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_live.npz")
+    path = os.path.join(here, "ref_live.npz")
+    np.savez_compressed(path, **out)
+    print("wrote", path, os.path.getsize(path), "bytes")
+    out = {}
+    preprocess(out)
+    path = os.path.join(here, "preprocess_ref.npz")
     np.savez_compressed(path, **out)
     print("wrote", path, os.path.getsize(path), "bytes")
 

@@ -57,8 +57,14 @@ def check_parity(logits, probs, idx, ref_logits, ref_probs, k=5, max_tol=1.25e-3
     return re
 
 
-@pytest.mark.parametrize("cfg", ["micro", "micro14", "tiny", "base"])
-def test_logits_and_topk_match_golden(cfg):
+@pytest.mark.parametrize("cfg,cta_group", [pytest.param(c, 2, id=c) for c in ("micro", "micro14", "tiny", "base")] +
+                         [pytest.param(c, 1, id=c + "-cg1") for c in ("micro", "tiny")])
+def test_logits_and_topk_match_golden(cfg, cta_group, monkeypatch):
+    """cta_group 1: VITB200_CTA_GROUP=1 at model creation runs every GEMM as its 1-CTA instantiation."""
+    if cta_group == 1:
+        monkeypatch.setenv("VITB200_CTA_GROUP", "1")
+    else:
+        monkeypatch.delenv("VITB200_CTA_GROUP", raising=False)
     g = np.load(os.path.join(GOLD, f"{cfg}_f16.npz"))
     m = eng.vit_model_load(model_path(cfg, "f16"), 0, 8)
     imgs = gf.synthetic_images(int(g["n_images"]), m.img_size, seed=int(g["image_seed"]))
@@ -256,11 +262,12 @@ def test_loader_rejects_wrong_shapes_and_duplicate_names():
     m2.close()
 
 
-@pytest.mark.parametrize("classes", [10, 1001, 21843])
+@pytest.mark.parametrize("classes", [10, 1001, 21843, 57857])
 def test_class_counts_that_are_not_a_multiple_of_four(classes, tmp_path):
     """ImageNet-21k heads have 21843 classes (the reference runs them); the head GEMM pads the class count to a multiple of 4
     internally (zero weight rows through TMA out-of-bounds fill, zero bias) and every output stays dense [batch][num_classes].
-    21843 floats also exceed the 48 KB default of the soft-max kernel's dynamic shared memory (opt-in up to 227 KB)."""
+    21843 floats also exceed the 48 KB default of the soft-max kernel's dynamic shared memory (opt-in up to 227 KB); 57857 floats
+    exceed that limit too, so the soft-max works on its row in global scratch."""
     path = str(tmp_path / f"micro-c{classes}.gguf")
     gf.write_synthetic(path, "micro", 1, classes=classes, seed=5)
     vf = gf.read(path)
@@ -388,31 +395,37 @@ def test_reference_cli_runs_unmodified_on_the_b200_engine(tmp_path):
         assert abs(float(g.split(":")[1]) - float(w.split(":")[1])) <= 0.011           # printed with %.2f
 
 
-@pytest.mark.skipif(not ref.available(), reason="oracle/_ref not shipped")
+PREPROCESS_REF = np.load(os.path.join(GOLD, "preprocess_ref.npz"))   # the reference's resizes (tests/golden/make_golden_ref.py)
+
+
 @pytest.mark.parametrize("bilinear", [False, True])
 def test_gpu_preprocess_matches_reference_bit_for_bit(bilinear):
     """SURVEY.md 8(f) rank 1: vit_image_preprocess on the GPU (bicubic default / bilinear), including the reference's quirks
-    (no half-pixel offset in bicubic, clamp-to-edge, double-precision cubic coefficients, round-to-u8 before normalising)."""
-    rng = np.random.default_rng(2)
-    sizes = [(300, 280), (224, 224), (97, 131), (512, 333), (64, 640)]  # (ny, nx): down-, identity-, up-scaling, odd aspect
-    imgs = [rng.integers(0, 256, size=(ny, nx, 3), dtype=np.uint8) for ny, nx in sizes]
-    # a smooth image too (random noise alone under-samples the interpolation arithmetic)
-    yy, xx = np.mgrid[0:400, 0:300]
-    imgs.append(np.stack([(127 + 120 * np.sin(xx / 17.0)), (127 + 120 * np.cos(yy / 23.0)), ((xx + yy) % 256)], -1).astype(np.uint8))
-    path = model_path("tiny", "f16")
-    rm = ref.RefModel(path)
-    m = eng.vit_model_load(path, 0, 8)
-    got, _, _, _, _ = eng.vit_image_preprocess_predict(m, imgs, bilinear=bilinear, predict=False)
-    for b, im in enumerate(imgs):
-        want = rm.preprocess(im, bilinear=bilinear)
-        mism = (got[b] != want)
-        # the normalised values are (u8 - mean)/std: any difference is a whole u8 level.  Bicubic (the reference default)
-        # reproduces the compiled reference's fused multiply-adds; in the bilinear path gcc fused the three unrolled channel
-        # iterations differently from each other, which is not replicated: a few values per 10^4 land one level off.
-        assert mism.mean() <= (5e-4 if bilinear else 2e-5), (b, im.shape, float(mism.mean()))
-        assert np.abs(got[b] - want).max() <= 1.01 / 57.0
-    m.close()
-    rm.close()
+    (no half-pixel offset in bicubic, clamp-to-edge, double-precision cubic coefficients, round-to-u8 before normalising), against
+    the reference's own output for down-, identity- and up-scaling, odd aspect ratios, single pixels, rows and columns, resized to
+    S = 64, 56 and 224.  All inputs of one S go through one call (mixed sizes in one staging buffer), a second call uses the other
+    pipeline slot, and one image at a time must give the same result."""
+    imgs = gf.preprocess_test_images()
+    mode = "bilinear" if bilinear else "bicubic"
+    mean = np.array([123.675, 116.280, 103.530], np.float32)
+    std = np.array([58.395, 57.120, 57.375], np.float32)
+    for cfg, S in (("micro", 64), ("micro14", 56), ("tiny", 224)):
+        res = PREPROCESS_REF[f"{mode}_{S}"]
+        m = eng.vit_model_load(model_path(cfg, "f16"), 0, len(imgs))
+        got = eng.vit_image_preprocess_predict(m, imgs, bilinear=bilinear, predict=False)[0]
+        again = eng.vit_image_preprocess_predict(m, imgs, bilinear=bilinear, predict=False)[0]
+        assert np.array_equal(again, got)
+        for b, im in enumerate(imgs):
+            levels = (rs.preprocess_levels(im, S, bilinear).astype(np.int16) + res[b]).astype(np.uint8)
+            want = (levels.astype(np.float32) - mean) / std
+            mism = got[b] != want
+            # the normalised values are (u8 - mean)/std: any difference is a whole u8 level.  Both modes reproduce the compiled
+            # reference's fused multiply-adds
+            assert mism.mean() <= 2e-5, (S, b, im.shape, float(mism.mean()))
+            assert np.abs(got[b] - want).max() <= 1.01 / 57.0, (S, b, im.shape)
+            alone = eng.vit_image_preprocess_predict(m, [im], bilinear=bilinear, predict=False)[0]
+            assert np.array_equal(alone[0], got[b]), (S, b, im.shape)
+        m.close()
 
 
 def test_forward_u8_end_to_end_vs_reference_pipeline():

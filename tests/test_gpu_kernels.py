@@ -29,8 +29,24 @@ CASES = [
 ]
 
 
-@pytest.mark.parametrize("M,N,K,epi", CASES)
-def test_gemm_against_numpy(M, N, K, epi):
+def with_cta_groups(cases):
+    """Every case with the default CTA pairs (ids as before) and with VITB200_CTA_GROUP=1 (id suffix -cg1), the 1-CTA
+    instantiation of every epilogue."""
+    ids = ["-".join(map(str, c)) for c in cases]
+    return ([pytest.param(*c, 2, id=i) for c, i in zip(cases, ids)] +
+            [pytest.param(*c, 1, id=i + "-cg1") for c, i in zip(cases, ids)])
+
+
+def set_cta_group(monkeypatch, cta_group):
+    if cta_group == 1:
+        monkeypatch.setenv("VITB200_CTA_GROUP", "1")
+    else:
+        monkeypatch.delenv("VITB200_CTA_GROUP", raising=False)
+
+
+@pytest.mark.parametrize("M,N,K,epi,cta_group", with_cta_groups(CASES))
+def test_gemm_against_numpy(M, N, K, epi, cta_group, monkeypatch):
+    set_cta_group(monkeypatch, cta_group)
     rng = np.random.default_rng(M * 7 + N * 3 + K + epi)
     A = rng.standard_normal((M, K)).astype(np.float16)
     W = (rng.standard_normal((N, K)) * 0.05).astype(np.float16)
@@ -50,10 +66,11 @@ def test_gemm_against_numpy(M, N, K, epi):
         assert (out != ref).mean() < 0.02
 
 
-@pytest.mark.parametrize("M,N,K", [(300, 576, 192), (197 * 3, 2304, 768), (129, 384, 192)])
-def test_gemm_split_precision_epilogue(M, N, K):
+@pytest.mark.parametrize("M,N,K,cta_group", with_cta_groups([(300, 576, 192), (197 * 3, 2304, 768), (129, 384, 192)]))
+def test_gemm_split_precision_epilogue(M, N, K, cta_group, monkeypatch):
     """EPI_BIAS_F16_HILO (the qkv GEMM in front of the tcgen05 attention): hi = f16(x), lo = f16(x - hi); hi + lo must carry the
     f32 result to ~2^-21 relative (2^-24 absolute once lo is subnormal), i.e. only fp32 accumulation-order noise remains."""
+    set_cta_group(monkeypatch, cta_group)
     rng = np.random.default_rng(M + N + K)
     A = rng.standard_normal((M, K)).astype(np.float16)
     W = (rng.standard_normal((N, K)) * 0.05).astype(np.float16)

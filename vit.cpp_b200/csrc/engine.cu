@@ -425,8 +425,10 @@ int upload_linear(vitb200_engine *e, const vitb200_tensor *t, int n, const std::
     return make_tmap(&L->tm, L->w, (uint64_t)n_out, (uint64_t)ld, (uint64_t)ld, (uint32_t)(L->bn / e->cta_group));
 }
 
-// dynamic shared memory the soft-max kernel may use for its working row (227 KB per CTA minus its static arrays)
-constexpr size_t kSoftmaxSmemMax = 232448 - 1024;
+// dynamic shared memory the soft-max kernel may use for its working row (227 KB per CTA minus room for its static arrays); the
+// launch needs the opt-in as soon as the row and those arrays exceed the 48 KB default
+constexpr size_t kSoftmaxStaticSmem = 1024;
+constexpr size_t kSoftmaxSmemMax = 232448 - kSoftmaxStaticSmem;
 
 enum ProfKind { PK_PATCH = 0, PK_QKV, PK_PROJ, PK_FC1, PK_FC2, PK_HEAD, PK_ATTN, PK_LN, PK_COUNT };
 
@@ -774,6 +776,33 @@ int launch_attention(vitb200_engine *e, int B, cudaStream_t s)
     return launch_attention_t<8>(e, B, s);
 }
 
+// floats of global scratch the soft-max needs for R rows of C classes: none while a row fits in shared memory
+size_t softmax_scratch_floats(int R, int C) { return (size_t)C * sizeof(float) > kSoftmaxSmemMax ? (size_t)R * C : 0; }
+
+// The soft-max / top-k launch of the forward (and of vitb200_test_softmax_topk): one CTA per row of lg ([R][ldl]); the working row
+// lives in dynamic shared memory while C floats fit in kSoftmaxSmemMax, and otherwise in `scratch` (softmax_scratch_floats(R, C)
+// floats; row r at scratch + r * C).
+int launch_softmax_topk(const float *lg, int ldl, float *probs, int32_t *idx, float *val, int R, int C, int k, float *scratch, cudaStream_t s)
+{
+    const size_t row_bytes = (size_t)C * sizeof(float);
+    const bool global_row = row_bytes > kSoftmaxSmemMax;
+    if (global_row && !scratch) return fail("soft-max over %d classes needs a global scratch row", C);
+    if (!global_row && row_bytes + kSoftmaxStaticSmem > 48 * 1024) // the static arrays count against the default too
+    {
+        static bool attr_set[64] = {}; // per device
+        int dev = 0;
+        CUDA_TRY(cudaGetDevice(&dev));
+        if (!attr_set[dev & 63])
+        {
+            CUDA_TRY(cudaFuncSetAttribute(softmax_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSoftmaxSmemMax));
+            attr_set[dev & 63] = true;
+        }
+    }
+    softmax_topk_kernel<<<R, 256, global_row ? 0 : row_bytes, s>>>(lg, ldl, probs, idx, val, C, k, global_row ? scratch : nullptr);
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
 // D2H helpers for the debug taps
 int tap_f32(float *dst, const float *src, size_t n, cudaStream_t s)
 {
@@ -949,10 +978,7 @@ int run_forward(vitb200_engine *e, const float *d_images, int B, float *d_probs,
         CUDA_TRY(cudaMemcpy2DAsync(d_logits, (size_t)C * 4, lg, (size_t)Cp * 4, (size_t)C * 4, (size_t)R, cudaMemcpyDeviceToDevice, s));
     if (d_probs || (k > 0 && (d_topk_idx || d_topk_val)))
     {
-        const size_t row_bytes = (size_t)C * sizeof(float);
-        float *scratch = row_bytes > kSoftmaxSmemMax ? e->d_sm_scratch : nullptr;
-        softmax_topk_kernel<<<R, 256, scratch ? 0 : row_bytes, s>>>(lg, Cp, d_probs, d_topk_idx, d_topk_val, C, k, scratch);
-        CUDA_TRY(cudaGetLastError());
+        if (launch_softmax_topk(lg, Cp, d_probs, d_topk_idx, d_topk_val, R, C, k, e->d_sm_scratch, s)) return 1;
         e->launches++;
     }
     return 0;
@@ -1133,12 +1159,9 @@ static int create_impl(const vitb200_hparams *hp, const vitb200_tensor *t, int n
         return bail(1);
     e->d_img_slot[0] = e->d_img; e->d_probs_slot[0] = e->d_probs;
     {
-        // soft-max working row: dynamic shared memory up to the per-CTA limit (opt-in above 48 KB), global scratch beyond it
-        const size_t row_bytes = (size_t)hp->num_classes * sizeof(float);
-        if (row_bytes > kSoftmaxSmemMax) { if (dev_alloc(e, &e->d_sm_scratch, R * hp->num_classes)) return bail(1); }
-        else if (row_bytes > 48 * 1024 &&
-                 cudaFuncSetAttribute(softmax_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSoftmaxSmemMax) != cudaSuccess)
-            return bail(fail("cudaFuncSetAttribute(softmax_topk_kernel) failed"));
+        // soft-max working rows in global memory when a row does not fit in shared memory (launch_softmax_topk)
+        const size_t n_scratch = softmax_scratch_floats((int)R, hp->num_classes);
+        if (n_scratch && dev_alloc(e, &e->d_sm_scratch, n_scratch)) return bail(1);
     }
     e->d_topk_idx_slot[0] = e->d_topk_idx; e->d_topk_val_slot[0] = e->d_topk_val;
     if (dev_alloc(e, &e->d_img_slot[1], B * img_elems) || dev_alloc(e, &e->d_probs_slot[1], R * hp->num_classes) ||
@@ -1719,6 +1742,36 @@ int vitb200_test_layernorm(int device, int rows, int D, const float *x, const fl
     cudaFree(dx); cudaFree(dw); cudaFree(db); cudaFree(dy);
     return rc;
     VB_NOEXCEPT_END((void)0)
+}
+
+// Stand-alone run of the final soft-max + top-k through the forward's own launcher (launch_softmax_topk): logits [R][ldl] f32, of which
+// the first C columns of every row are read -> probs [R][C], idx / val [R][k].
+int vitb200_test_softmax_topk(int device, int R, int C, int ldl, const float *logits, int k, float *probs, int32_t *idx, float *val)
+{
+    if (!logits || !probs || R < 1 || C < 1 || ldl < C || k < 0 || k > 16 || (k > 0 && (!idx || !val))) return fail("bad argument");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("no CUDA device: the vit.cpp_b200 forward path has no CPU fallback");
+    if (device < 0 || device >= ndev) return fail("device %d out of range (%d devices)", device, ndev);
+    CUDA_TRY(cudaSetDevice(device));
+    float *dl = nullptr, *dp = nullptr, *dv = nullptr, *dscr = nullptr;
+    int32_t *di = nullptr;
+    const size_t n_scratch = softmax_scratch_floats(R, C);
+    int rc = 1;
+    do
+    {
+        if (cudaMalloc(&dl, (size_t)R * ldl * 4) || cudaMalloc(&dp, (size_t)R * C * 4) || cudaMalloc(&di, (size_t)R * (k ? k : 1) * 4) ||
+            cudaMalloc(&dv, (size_t)R * (k ? k : 1) * 4) || (n_scratch && cudaMalloc(&dscr, n_scratch * 4))) { fail("cudaMalloc failed"); break; }
+        if (cudaMemcpy(dl, logits, (size_t)R * ldl * 4, cudaMemcpyHostToDevice) != cudaSuccess) { fail("H2D failed"); break; }
+        if (launch_softmax_topk(dl, ldl, dp, k ? di : nullptr, k ? dv : nullptr, R, C, k, dscr, 0)) break;
+        cudaError_t err = cudaDeviceSynchronize();
+        if (err != cudaSuccess) { fail("soft-max kernel failed: %s", cudaGetErrorString(err)); break; }
+        if (cudaMemcpy(probs, dp, (size_t)R * C * 4, cudaMemcpyDeviceToHost) != cudaSuccess ||
+            (k && (cudaMemcpy(idx, di, (size_t)R * k * 4, cudaMemcpyDeviceToHost) != cudaSuccess ||
+                   cudaMemcpy(val, dv, (size_t)R * k * 4, cudaMemcpyDeviceToHost) != cudaSuccess))) { fail("D2H failed"); break; }
+        rc = 0;
+    } while (0);
+    cudaFree(dl); cudaFree(dp); cudaFree(di); cudaFree(dv); cudaFree(dscr);
+    return rc;
 }
 
 // q8_0 linear layer on the integer tensor cores (gemm_q8_tcgen05.cuh; prototype for BASELINE.json configs[4]): x [M][K] f32 is

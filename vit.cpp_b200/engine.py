@@ -85,6 +85,7 @@ def lib():
         L.vitb200_test_dequant.argtypes = [i32, vp, C.c_int64, vp]
         L.vitb200_test_gemm_q8.argtypes = [i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, i32, vp]
         L.vitb200_test_layernorm.argtypes = [i32, i32, i32, vp, vp, vp, C.c_float, vp]
+        L.vitb200_test_softmax_topk.argtypes = [i32, i32, i32, i32, vp, i32, vp, vp, vp]
         L.vitb200_test_attention.argtypes = [i32, i32, i32, i32, i32, vp, vp]
         L.vitb200_test_attention_hilo.argtypes = [i32, i32, i32, i32, vp, vp, vp]
         _lib = L
@@ -361,3 +362,16 @@ def test_layernorm(x, w, b, eps: float = 1e-6, device: int = 0):
     _check(lib().vitb200_test_layernorm(device, x.shape[0], x.shape[1], x.ctypes.data, w.ctypes.data, b.ctypes.data, eps, y.ctypes.data),
            "vitb200_test_layernorm")
     return y
+
+
+def test_softmax_topk(logits, C: int, k: int, device: int = 0):
+    """The final soft-max + top-k kernel alone (vitb200_test_softmax_topk): logits float32 [R][ldl] with ldl >= C (only the first C
+    columns are read).  Returns (probs [R][C] f32, idx [R][k] int32, val [R][k] f32)."""
+    lg = np.ascontiguousarray(logits, np.float32)
+    R, ldl = lg.shape
+    probs = np.empty((R, C), np.float32)
+    idx = np.empty((R, k), np.int32)
+    val = np.empty((R, k), np.float32)
+    _check(lib().vitb200_test_softmax_topk(device, R, C, ldl, lg.ctypes.data, k, probs.ctypes.data, idx.ctypes.data, val.ctypes.data),
+           "vitb200_test_softmax_topk")
+    return probs, idx, val
